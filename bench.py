@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- mel frames/sec of the fused STFT -> |.| -> mel -> dB hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path over one batch of synthetic waveforms.  Workload (N=1 and
 per rank for N>1, weak scaling): BASELINE.json configs[1] -- batch 256, mono, 22.05 kHz x 5 s,
@@ -15,6 +15,9 @@ Rank 0 prints ONE JSON line (contract in the task statement):
   cpu_baseline  the oracle's multi-threaded CPU port on the same workload, timed on rank 0
 ``--impl reference`` times that CPU port alone (the reference itself needs TensorFlow + librosa,
 which are not installable here; see DESIGN.md).
+``--dump-outputs DIR`` writes what the last timed step returned (rank 0's log-mel tensor) to
+DIR/logmel_db.npy, float32.  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -59,6 +62,7 @@ def select_config(name, rank, world):
         CFG['batch'] = hi - lo
         CFG['shard'] = [lo, hi]
     WORKLOAD = CFG['workload']
+DUMP_LIMIT = 60_000_000  # bytes of --dump-outputs, under 64 MB with the .npy header; beyond it, a sample of items
 PROFILE_EVERY = 8  # every 8th fused-kernel launch of the timed loop is bracketed by CUDA events (roofline.kernel_ms)
 N_SETS = 3  # rotating input/output sets: 3 x (113 MB in + 56 MB out) = 507 MB > 126 MB L2
 
@@ -142,6 +146,20 @@ class ClockSampler:
                 'samples': len(s)}
 
 
+def dump_outputs(out_dir, y):
+    """Write the device tensor `y` (batch first) to out_dir/logmel_db.npy as float32: whole if it fits in
+    DUMP_LIMIT, otherwise the batch items np.random.default_rng(0).choice(batch, n, replace=False) picks, in
+    increasing order, for the largest n that fits."""
+    import numpy as np
+    item_bytes = y[0].numel() * 4
+    if y.shape[0] * item_bytes > DUMP_LIMIT:
+        n = max(1, DUMP_LIMIT // item_bytes)
+        items = np.sort(np.random.default_rng(0).choice(y.shape[0], n, replace=False))
+        y = y[items.tolist()]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'logmel_db.npy'), y.float().cpu().numpy())
+
+
 def cpu_port(threads=None):
     import torch
     from oracle.fast_cpu import MelSpectrogramCPU
@@ -196,7 +214,13 @@ def main():
     ap.add_argument('--config', default='auto', choices=['auto', 'cfg2', 'cfg5'],
                     help='auto: cfg2 per rank below 8 ranks (weak scaling), cfg5 (batch 8192 sharded) on 8 ranks')
     ap.add_argument('--no-numa-bind', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the output of the last timed step to DIR/logmel_db.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the CUDA path\'s outputs (--impl b200)')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -321,6 +345,8 @@ def main():
     barrier()
     sampler.stop()
     _native.profile_enable(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs[(args.steps - 1) % N_SETS])
     ms_total = reduce_max(e0.elapsed_time(e1))
     launches = _native.launch_count() - n0
     kern_ms, kern_n = _native.profile_read()

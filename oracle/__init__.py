@@ -26,10 +26,10 @@ reference's layers and composed models return for 55 cases (``tests/golden/kapre
   reference's literal dB test matrix (``tests/test_backend.py:20-22``) and analytic known-answer
   tests (impulse, DC, bin-centred cosine, Parseval, STFT->ISTFT identity).
 
-In the build container (where /root/reference exists) ``tests/test_reference_fidelity.py`` additionally
-re-runs the comparison on random configurations (``make_golden_ref.py --fuzz``: STFT / mel factory outputs
-and which argument combinations raise) and compares constructor errors and ``get_config()`` of every layer
-mirror with the reference's classes (``tests/golden/check_api_fidelity.py``).
+``tests/test_reference_fidelity.py`` additionally holds the oracle to the reference's outputs on random
+STFT / mel configurations (including which argument combinations raise), and every layer mirror to the
+reference's constructor errors and ``get_config()``: answers of the reference's own classes recorded by
+``tests/golden/make_golden_fidelity.py`` in ``tests/golden/kapre_ref_fidelity.*``.
 
 See ``tests/golden/make_golden.py`` / ``make_golden_ref.py`` for the scripts that produced the committed fixtures.
 """

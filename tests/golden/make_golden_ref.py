@@ -196,54 +196,5 @@ def main():
     print('wrote %d cases, %.1f KiB' % (len(manifest), size / 1024.0))
 
 
-def fuzz(n, seed=0):
-    """Differential check on random configurations: the reference's STFT layer and mel factory (over the
-    stand-in) against the oracle, including which argument combinations raise.  Nothing is stored."""
-    sys.path.append(os.path.join(HERE, '..', '..'))
-    import oracle as O
-    rng = np.random.default_rng(seed)
-    bad = 0
-    for _ in range(n):
-        n_fft = int(rng.choice([64, 100, 256, 500, 512]))
-        win = int(rng.integers(2, n_fft + 1)) if rng.random() < 0.5 else None
-        hop = int(rng.integers(1, n_fft + 1)) if rng.random() < 0.7 else None
-        wname = rng.choice([None, 'hann_window', 'hamming_window', 'kaiser_window', 'vorbis_window'])
-        wname = None if wname is None else str(wname)
-        pb, pe = bool(rng.random() < 0.5), bool(rng.random() < 0.5)
-        ifmt = str(rng.choice(['channels_first', 'channels_last', 'default']))
-        ofmt = str(rng.choice(['channels_first', 'channels_last', 'default']))
-        C, L = int(rng.integers(1, 4)), int(rng.integers(n_fft, 4 * n_fft + 50))
-        x = rng.uniform(-1, 1, size=(2, L, C) if ifmt != 'channels_first' else (2, C, L))
-        kw = dict(n_fft=n_fft, win_length=win, hop_length=hop, window_name=wname, pad_begin=pb, pad_end=pe,
-                  input_data_format=ifmt, output_data_format=ofmt)
-        try:
-            a = kapre.STFT(**kw)(x)
-        except Exception as e:  # noqa: BLE001
-            try:
-                O.stft_layer(x, **kw)
-                print('reference raised, oracle did not:', kw, repr(e)[:80])
-                bad += 1
-            except Exception:  # noqa: BLE001
-                pass
-            continue
-        b = O.stft_layer(x, **kw)
-        if a.shape != b.shape or (a.size and np.abs(a - b).max() > 1e-9 * max(1.0, np.abs(a).max())):
-            print('STFT mismatch:', kw)
-            bad += 1
-        if a.size and rng.random() < 0.4:
-            mk = dict(kw, sample_rate=int(rng.choice([8000, 16000, 22050])), n_mels=int(rng.integers(2, 40)),
-                      mel_htk=bool(rng.random() < 0.5), return_decibel=bool(rng.random() < 0.7),
-                      db_dynamic_range=float(rng.choice([80.0, 30.0])))
-            a = KC.get_melspectrogram_layer(**mk)(x)
-            b = O.melspectrogram_layer(x, **mk)
-            if a.shape != b.shape or np.abs(a - b).max() > 1e-7 * max(1.0, np.abs(a).max()):
-                print('mel mismatch:', mk)
-                bad += 1
-    print('fuzz: %d configurations, %d disagreements' % (n, bad))
-    return bad
-
-
 if __name__ == '__main__':
-    if len(sys.argv) > 2 and sys.argv[1] == '--fuzz':
-        sys.exit(1 if fuzz(int(sys.argv[2])) else 0)
     main()

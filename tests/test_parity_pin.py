@@ -90,9 +90,9 @@ def test_reference_cases_regenerate_with_real_tensorflow_and_librosa():
     if importlib.util.find_spec('tensorflow') is None or importlib.util.find_spec('librosa') is None:
         pytest.skip('tensorflow / librosa not installed: the committed fixtures come from the stand-in '
                     '(tests/golden/tf_standin.py); run tests/golden/regen_with_real_libs.py where they exist')
-    ref_root = os.environ.get('KAPRE_REFERENCE_ROOT', '/root/reference')
-    if not os.path.isdir(os.path.join(ref_root, 'kapre')):
-        pytest.skip('reference sources not present at %s' % ref_root)
+    ref_root = os.environ.get('KAPRE_REFERENCE_ROOT')
+    if not ref_root or not os.path.isdir(os.path.join(ref_root, 'kapre')):
+        pytest.skip('KAPRE_REFERENCE_ROOT does not name a directory holding the kapre 0.4.0 package')
     out = subprocess.run([sys.executable, os.path.join(HERE, 'golden', 'regen_with_real_libs.py'), '--check'],
                          capture_output=True, text=True)
     assert out.returncode == 0, out.stdout + out.stderr
