@@ -159,6 +159,60 @@ int kapre_frame(const float* x_dev, const kapre_wave_desc* x_desc, int frame_len
 int kapre_energy(const float* x_dev, const kapre_wave_desc* x_desc, int frame_length, int hop_length, int pad_end,
                  float pad_value, float scale, float* out_dev, const kapre_wave_desc* out_desc, void* stream);
 
+/* ---- backward: vector-Jacobian products of the hot-path layers -------------------------------------------------
+ * The rules restate TensorFlow's registered gradients of the ops the reference calls (RFFT / IRFFT, ComplexAbs,
+ * MatMul, Log, Maximum, Max, tf.signal.frame's scatter-add, tf.pad's slice).  A complex gradient G is
+ * dL/dRe + i dL/dIm.  Windows, filterbanks and dual windows are constants.  Every input is described by element
+ * strides; any stride may be 0 (the gradient of a sum arrives as an expanded tensor).  Results are deterministic:
+ * the same inputs give the same bits on every run. */
+
+/* VJP of kapre_stft_forward(KAPRE_OUT_COMPLEX): complex64 gradient of the (batch, channels, frames, n_fft/2+1)
+ * spectrum -> float32 gradient of the waveform, `grad_x_desc->length` samples (frames must equal
+ * kapre_stft_num_frames(plan, length, pad_begin, pad_end)).  Frame t contributes
+ * w[n] * sum_{k <= n_fft/2} Re(G_t[k] e^{+2 pi i k n / n_fft}) at padded sample t*hop + n, n < min(win_length, n_fft);
+ * the pad_begin prefix is dropped and samples no frame covers get 0.  n_fft in {256,512,1024,2048}: the streaming
+ * inverse-FFT kernel of kapre_istft_inverse with the window n_fft/2 * w; any other n_fft: a direct O(n_fft) sum per
+ * sample and frame.  No workspace.  grad_spec and grad_x must not overlap. */
+int kapre_stft_backward(const kapre_stft_plan* plan, const void* grad_spec_dev, int batch, int channels, int frames,
+                        const kapre_spec_desc* grad_spec_desc, int pad_begin, int pad_end, float* grad_x_dev,
+                        const kapre_wave_desc* grad_x_desc, void* stream);
+
+/* VJP of kapre_istft_inverse: float32 gradient of the (batch, channels, (frames-1)*hop+win_length) waveform ->
+ * complex64 gradient of the spectrum, G_t[k] = (c_k / n_fft) sum_{n < min(win_length, n_fft)} dual[n] g[t*hop + n]
+ * e^{-2 pi i k n / n_fft} with c_0 = c_{n_fft/2} = 1 (n_fft/2 for even n_fft only), c_k = 2 otherwise; Im G[0] and
+ * Im G[n_fft/2] are 0.  Runs kapre_stft_forward(KAPRE_OUT_COMPLEX) with a forward plan the inverse plan holds
+ * (window 2/n_fft * dual), then halves the edge bins: every n_fft is served.  No workspace; no overlap. */
+int kapre_istft_backward(const kapre_istft_plan* plan, const float* grad_y_dev, const kapre_wave_desc* grad_y_desc,
+                         void* grad_spec_dev, int frames, const kapre_spec_desc* grad_spec_desc, void* stream);
+
+/* VJP of the chain |X| [-> filterbank] [-> dB] at the complex64 STFT X (batch, channels, frames, n_freq), `mode` one
+ * of KAPRE_OUT_MAG, _MAG_DB, _FB, _FB_DB (KAPRE_OUT_MAG alone is kapre.Magnitude's VJP).  grad: float32 upstream
+ * gradient of the chain's (batch, channels, frames, K) output, K = n_freq or fb's band count; y (decibel modes):
+ * that forward output.  Writes the complex64 gradient of X: G = g_mag X / |X| (0 where |X| = 0) with
+ * g_mag = g_fb fb^T and the decibel rule of kapre_magnitude_to_decibel_backward per batch item.
+ * workspace_dev (decibel modes): >= 1056 * batch + 16 bytes, zero on entry, left zero (self-cleaning).
+ * grad_x may alias x exactly (same pointer and strides: in place); no other overlap. */
+int kapre_spectral_backward(const kapre_filterbank* fb, int mode, const void* x_dev, int batch, int channels, int frames,
+                            int n_freq, const kapre_spec_desc* x_desc, const float* grad_dev,
+                            const kapre_spec_desc* grad_desc, const float* y_dev, const kapre_spec_desc* y_desc,
+                            const kapre_db_cfg* db, void* workspace_dev, void* grad_x_dev,
+                            const kapre_spec_desc* grad_x_desc, void* stream);
+
+/* VJP of kapre_magnitude_to_decibel on contiguous (n_items, item_size) x (its input) and y (its output); the upstream
+ * gradient has element strides (grad_item_stride, grad_elem_stride).  With l = 10 log10(max(x, amin)) - c,
+ * m = max_item(l), thr = m - dynamic_range:
+ *   dL/dl_i = g_i [l_i >= thr] + [l_i == m] sum_j g_j [l_j < thr] / #{l_j == m}   (the clamp's gradient goes to the
+ *   item maximum, ties split it equally),  dL/dx_i = dL/dl_i 10 / (ln 10 max(x_i, amin)) [x_i >= amin].
+ * Clamped elements are read from y: an item's clamp binds when min(y) <= max(y) - dynamic_range within a few float32
+ * ulps, and then exactly the elements with y_i == min(y) are clamped (an unclamped l_i within float32 rounding of thr
+ * counts as clamped).  Two launches: per-item statistics in fixed order (last-CTA combine), then the element rule.
+ * workspace_dev: >= 1056 * n_items + 16 bytes, zero on entry, left zero.  grad_x may alias grad when both are
+ * contiguous; no other overlap. */
+int kapre_magnitude_to_decibel_backward(const float* x_dev, const float* y_dev, const float* grad_dev,
+                                        int64_t grad_item_stride, int64_t grad_elem_stride, float* grad_x_dev,
+                                        int64_t n_items, int64_t item_size, const kapre_db_cfg* db, void* workspace_dev,
+                                        void* stream);
+
 /* ---- misc ---------------------------------------------------------------------------------- */
 const char* kapre_last_error(void);
 int kapre_version(void);

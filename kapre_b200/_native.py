@@ -57,6 +57,14 @@ SYMBOLS = [
     ('kapre_energy', c_int, [c_void_p, POINTER(WaveDesc), c_int, c_int, c_int, c_float, c_float, c_void_p, POINTER(WaveDesc), c_void_p]),
     ('kapre_concat_frequency_map', c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int, c_void_p]),
     ('kapre_spec_augment', c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p, c_int, c_float, c_void_p]),
+    ('kapre_stft_backward', c_int, [c_void_p, c_void_p, c_int, c_int, c_int, POINTER(SpecDesc), c_int, c_int, c_void_p,
+                                    POINTER(WaveDesc), c_void_p]),
+    ('kapre_istft_backward', c_int, [c_void_p, c_void_p, POINTER(WaveDesc), c_void_p, c_int, POINTER(SpecDesc), c_void_p]),
+    ('kapre_spectral_backward', c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, POINTER(SpecDesc), c_void_p,
+                                        POINTER(SpecDesc), c_void_p, POINTER(SpecDesc), POINTER(DbCfg), c_void_p, c_void_p,
+                                        POINTER(SpecDesc), c_void_p]),
+    ('kapre_magnitude_to_decibel_backward', c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64,
+                                                    c_int64, POINTER(DbCfg), c_void_p, c_void_p]),
     ('kapre_last_error', c_char_p, []),
     ('kapre_version', c_int, []),
     ('kapre_launch_count', c_uint64, []),

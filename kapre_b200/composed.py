@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from . import backend, ops
+from . import autograd, backend, ops
 from .backend import _CH_DEFAULT_STR, _CH_FIRST_STR, _CH_LAST_STR
 from .time_frequency import (STFT, ApplyFilterbank, InverseSTFT, Layer, Magnitude, MagnitudeToDecibel, Phase,
                              get_registered_object)
@@ -116,8 +116,11 @@ class Sequential(Layer):
                 if dbl.dynamic_range <= 0:
                     raise ValueError('dynamic_range must be positive, got: %s' % (dbl.dynamic_range,))
                 db = (dbl.ref_value, dbl.amin, dbl.dynamic_range)
-            x = ops.stft_forward(x, stft.plan, stft.input_data_format, stft.output_data_format, stft.pad_begin,
-                                 stft.pad_end, mode, fbl.fb if fbl is not None else None, db)
+            if autograd.wants_grad(x):
+                x = autograd.FusedSpectrogramFn.apply(x, stft, mode, fbl.fb if fbl is not None else None, db)
+            else:
+                x = ops.stft_forward(x, stft.plan, stft.input_data_format, stft.output_data_format, stft.pad_begin,
+                                     stft.pad_end, mode, fbl.fb if fbl is not None else None, db)
             start = n
         for layer in self.layers[start:]:
             x = layer.call(x)

@@ -243,6 +243,7 @@ struct KbIdftParams {
     long long y_sb, y_sc, y_sl;
     int n_tiles_s;            // ceil(out_len / (32 * n_warps))
     int n_warps;
+    int y_off, edge2;         // STFT adjoint only (see KbIstftParams); zero for the inverse STFT
 };
 
 #if defined(KB_HOST_EMU)
@@ -274,7 +275,7 @@ __device__ __forceinline__ void kb_idft_cta(const KbIdftParams& p, char* smem, i
         KB_PHASE_BEGIN
             (void)R;
             const int s = ts * kb_nt + tid;
-            if (s < p.out_len) {
+            if (s >= p.y_off && s < p.out_len) {
                 float acc = 0.0f;
                 int t_hi = s / p.hop;
                 if (t_hi > p.T - 1) t_hi = p.T - 1;
@@ -282,21 +283,21 @@ __device__ __forceinline__ void kb_idft_cta(const KbIdftParams& p, char* smem, i
                     const int n = s - t * p.hop;
                     if (n >= p.win) break;
                     const float2* Xf = Xsig + (long long)t * p.x_st;
-                    float sum = Xf[0].x;
+                    float sum = p.edge2 ? 2.0f * Xf[0].x : Xf[0].x;
                     int r = n % N;
                     const int step = r;
                     for (int k = 1; k < F; ++k) {
                         const float2 xv = Xf[(long long)k * p.x_sk];
                         const cpx w = tw_s[r];
                         const bool nyq = ((N & 1) == 0) && (k == F - 1);
-                        if (nyq) sum += xv.x * w.re;
+                        if (nyq) sum += (p.edge2 ? 2.0f * xv.x : xv.x) * w.re;
                         else sum += 2.0f * (xv.x * w.re - xv.y * w.im);
                         r += step;
                         if (r >= N) r -= N;
                     }
                     acc += sum * p.dualn[n];
                 }
-                p.y[(long long)b * p.y_sb + (long long)c * p.y_sc + (long long)s * p.y_sl] = acc;
+                p.y[(long long)b * p.y_sb + (long long)c * p.y_sc + (long long)(s - p.y_off) * p.y_sl] = acc;
             }
         KB_PHASE_END
     }

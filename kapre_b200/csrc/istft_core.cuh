@@ -318,7 +318,8 @@ KB_FN void kb_istft2_prefetch(KbThreadRegs& R, const KbIstftParams& p, const flo
     }
 }
 
-template <int Q>
+// ADJ: the STFT adjoint (kapre_stft_backward) -- honours p.y_off and p.edge2; the inverse instantiation ignores both.
+template <int Q, bool ADJ = false>
 #if defined(KB_HOST_EMU)
 inline void kb_istft2_cta(const KbIstftParams& p, char* smem, int cta, int n_cta)
 #else
@@ -371,9 +372,12 @@ __device__ __forceinline__ void kb_istft2_cta(const KbIstftParams& p, char* smem
         const int h0 = tt * seg;                 // first output hop of the tile
         const int tf0 = h0 - Rm1;                // first (possibly negative) frame transformed
         const float2* Xsig = p.X + (long long)b * p.x_sb + (long long)c * p.x_sc;
-        float* ysig = p.y + (long long)b * p.y_sb + (long long)c * p.y_sc;
-        const long long s_lo = (long long)h0 * H;
+        // (shifted by y_off: sample s is stored at y[s - y_off]; only s >= y_off is stored)
+        const int y_off = ADJ ? p.y_off : 0;
+        float* ysig = p.y + (long long)b * p.y_sb + (long long)c * p.y_sc - (long long)y_off * p.y_sl;
+        long long s_lo = (long long)h0 * H;
         long long s_hi = s_lo + (long long)seg * H;
+        if (s_lo < y_off) s_lo = y_off;
         if (s_hi > p.out_len) s_hi = p.out_len;
 
         KB_PHASE_BEGIN
@@ -400,7 +404,10 @@ __device__ __forceinline__ void kb_istft2_cta(const KbIstftParams& p, char* smem
                     const int k = lane + 32 * i;
                     cpx a = R.v[e];
                     cpx bq = R.v[16 + e];
-                    if (k == 0) { a.im = 0.0f; bq.im = 0.0f; }  // C2R ignores Im of DC / Nyquist
+                    if (k == 0) {                               // C2R ignores Im of DC / Nyquist
+                        a.im = 0.0f; bq.im = 0.0f;
+                        if (ADJ && p.edge2) { a.re *= 2.0f; bq.re *= 2.0f; }
+                    }
                     const cpx W = twn_s[k];
                     // packed arithmetic: E = a + conj(b), D = a - conj(b), O = conj(W) D;
                     // conj(2 Z[k]) = conj(E + i O), conj(2 Z[P-k]) = E - i O

@@ -22,6 +22,7 @@
 #include "mr_core.cuh"
 #include "tc_dft.cuh"
 #include "tc_mel.cuh"
+#include "grad_core.cuh"
 
 // ------------------------------------------------------------------------------------------
 // error handling
@@ -145,6 +146,39 @@ __global__ void __launch_bounds__(512) kb_mr_kernel(const __grid_constant__ KbMr
 __global__ void __launch_bounds__(KB_MAX_WARPS * 32) kb_idft_kernel(const __grid_constant__ KbIdftParams p) {
     extern __shared__ __align__(16) char kb_smem[];
     kb_idft_cta(p, kb_smem, (int)blockIdx.x, (int)gridDim.x);
+}
+
+// ---- backward kernels (grad_core.cuh) ----
+__global__ void __launch_bounds__(KB_DBS_THREADS) kb_dbstat_kernel(const __grid_constant__ KbDbStatParams p) {
+    __shared__ __align__(16) char kb_smem[KB_DBS_THREADS * sizeof(KbDbStats) + 16];
+    kb_dbstat_cta(p, kb_smem, (int)blockIdx.x, (int)gridDim.x);
+}
+
+__global__ void __launch_bounds__(KB_MAX_WARPS * 32) kb_specvjp_kernel(const __grid_constant__ KbSpecVjpParams p) {
+    extern __shared__ __align__(16) char kb_smem[];
+    kb_specvjp_cta(p, kb_smem, (int)blockIdx.x, (int)gridDim.x);
+}
+
+// Stand-alone MagnitudeToDecibel VJP, element-wise on contiguous (n_items, item_size) x / y; g has (item, element) strides.
+__global__ void kb_db_backward_kernel(const float* __restrict__ x, const float* __restrict__ y, const float* __restrict__ g,
+                                      long long g_si, long long g_se, float* __restrict__ dx, long long item_size, long long n,
+                                      const KbDbStats* __restrict__ stats, float amin) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const long long item = i / item_size, e = i - item * item_size;
+        dx[i] = kb_db_dl(stats[item], y[i], g[item * g_si + e * g_se]) * kb_db_dx(x[i], amin);
+    }
+}
+
+// InverseSTFT VJP fix-up: the forward STFT of the upstream gradient carries weight 2/N on every bin; bins 0 and N/2
+// (even N) of the irfft count once, so they are halved, and their imaginary parts (which irfft ignores) get 0.
+__global__ void kb_istft_grad_edges_kernel(float2* __restrict__ G, long long sb, long long sc, long long st, long long sk,
+                                           int C, int T, long long n_frames, int last, int even) {
+    for (long long fr = (long long)blockIdx.x * blockDim.x + threadIdx.x; fr < n_frames; fr += (long long)gridDim.x * blockDim.x) {
+        const long long t = fr % T, bc = fr / T;
+        float2* Gf = G + (bc / C) * sb + (bc % C) * sc + t * st;
+        Gf[0] = make_float2(0.5f * Gf[0].x, 0.0f);
+        if (even) Gf[(long long)last * sk] = make_float2(0.5f * Gf[(long long)last * sk].x, 0.0f);
+    }
 }
 
 // Dynamic-range clamp, kapre/backend.py:190-192: y = max(y, max_item(y) - dynamic_range).
@@ -372,6 +406,10 @@ struct kapre_stft_plan {
     float* w = nullptr;       // generic path: window[0, win_eff)
     float2* tw = nullptr;     // generic path: exp(-2 pi i r / n_fft)
     int win_eff;
+    // STFT adjoint (kapre_stft_backward): the inverse kernels with the window n_fft/2 * w in place of the dual window
+    float* adj = nullptr;     // streaming body: kb_make_dual(n_fft/2 * window)
+    float* adj_dn = nullptr;  // direct body: (n_fft/2 * window) / n_fft = window / 2
+    float2* adj_tw = nullptr; // direct body: exp(+2 pi i r / n_fft)
     // tensor-core path (tc_mel.cuh; n_fft = win_length = 1024, cosine-sum window a - b cos): constant operands
     double win_a = 0.0, win_b = 0.0;
     float* tc_f1 = nullptr;   // stage-1 matrix hi/lo
@@ -447,6 +485,7 @@ struct kapre_istft_plan {
     float2* twn = nullptr;
     float* dualn = nullptr;   // generic path: dual / n_fft
     float2* tw = nullptr;     // generic path: exp(+2 pi i r / n_fft)
+    kapre_stft_plan* grad = nullptr;   // VJP (kapre_istft_backward): forward STFT with the window 2/n_fft * dual
 };
 
 struct kapre_filterbank {
@@ -454,6 +493,8 @@ struct kapre_filterbank {
     DevInfo dev;
     KbBand* bands = nullptr;   // band-major form (stand-alone ApplyFilterbank kernel)
     float* w = nullptr;
+    KbBand* bandsT = nullptr;  // the same form of the transposed matrix (per bin: the bands it feeds), spectral VJP
+    float* wT = nullptr;
     int Q = 0;                 // chunk-list form for the fused kernel (n_freq == 32*Q + 1), else 0
     int n_chunks = 0;
     kb_f4* cw = nullptr;
@@ -628,18 +669,18 @@ static int kb_launch_stft(const KbStftParams& p, int grid, int smem, cudaStream_
     return kb_fail(KAPRE_E_INVALID, "bad mode");
 }
 
-template <int Q>
+template <int Q, bool ADJ>
 __global__ void __launch_bounds__(KB_ISTFT_MAX_WARPS * 32, 4) kb_istft2_kernel(const __grid_constant__ KbIstftParams p) {
     extern __shared__ __align__(128) char kb_smem[];
-    kb_istft2_cta<Q>(p, kb_smem, (int)blockIdx.x, (int)gridDim.x);
+    kb_istft2_cta<Q, ADJ>(p, kb_smem, (int)blockIdx.x, (int)gridDim.x);
 }
 
-template <int Q>
+template <int Q, bool ADJ = false>
 static int kb_launch_istft2(const KbIstftParams& p, int grid, int smem, cudaStream_t st) {
-    int rc = kb_set_smem(kb_istft2_kernel<Q>, smem);
+    int rc = kb_set_smem(kb_istft2_kernel<Q, ADJ>, smem);
     if (rc) return rc;
     KbProfScope prof(st);
-    kb_istft2_kernel<Q><<<grid, p.n_warps * 32, smem, st>>>(p);
+    kb_istft2_kernel<Q, ADJ><<<grid, p.n_warps * 32, smem, st>>>(p);
     KB_CUDA(cudaGetLastError());
     g_launches++;
     return 0;
@@ -654,6 +695,69 @@ static int kb_launch_istft(const KbIstftParams& p, int grid, int smem, cudaStrea
     KB_CUDA(cudaGetLastError());
     g_launches++;
     return 0;
+}
+
+
+// Launch configuration of the streaming inverse kernel (kb_istft2_cta) for `out_len` output samples: tiles of
+// seg = m * FR - (R - 1) output hops, m rounds of FR = NW * FPW frames each.  m is the round count that minimises
+// (waves of tiles over the resident CTAs) x (rounds per tile).  Fills the shape fields of *p; returns 1 when the tile
+// does not fit shared memory (the caller falls back), 0 on success, < 0 on error.
+static int kb_istft2_cfg(const DevInfo& dev, int Q, int n_fft, int hop, int win, int batch, int channels, int frames,
+                         long long out_len, KbIstftParams* pp, int* grid_out) {
+    const int FPW = 32 / Q;
+    const int R = (win + hop - 1) / hop;
+    const int NW = KB_ISTFT_MAX_WARPS, FR = NW * FPW;
+    const KbIstft2Smem L2 = kb_istft2_smem_layout(Q, n_fft, hop, win, NW);
+    if (L2.total > dev.smem_optin) return 1;
+    int bps = (228 * 1024) / (L2.total + 1024);
+    if (bps > 4) bps = 4;              // __launch_bounds__(128, 4)
+    if (bps < 1) bps = 1;
+    const long long slots = (long long)dev.sm_count * bps;
+    const long long hops = (out_len + hop - 1) / hop;
+    // rounds per tile: the most (<= 6: R - 1 halo frames per tile cost <= 6 %) that still leave about one tile per
+    // resident CTA.  Measured (profiles/r2_istft_streaming.md): at B256 x 5 s tiles of 6 rounds beat one wave of 28-round
+    // tiles by 6 % (the static tile walk balances per SM, not per CTA); at B128 x 1 s tiles of 3 rounds (512 tiles on
+    // 592 slots) beat 2 and 4.
+    // Floor: tiles long enough that the halo stays under ~20 % of the frames (hop << win: R is large).
+    int m_lo = (5 * (R - 1) + FR - 1) / FR;
+    if (m_lo < 1) m_lo = 1;
+    const int m_hi = m_lo > 6 ? m_lo : 6;
+    int best_m = m_lo, best_seg = m_lo * FR - (R - 1);
+    for (int m = m_hi; m >= m_lo; --m) {
+        const int seg = m * FR - (R - 1);
+        const long long nt = (long long)batch * channels * ((hops + seg - 1) / seg);
+        best_m = m; best_seg = seg;
+        if (nt * 100 >= slots * 85) break;
+    }
+    const int m_env = kb_env_int("KAPRE_B200_ISTFT2_M", 0);
+    if (m_env > 0 && m_env * FR - (R - 1) >= 1) { best_m = m_env; best_seg = m_env * FR - (R - 1); }
+    KbIstftParams& p = *pp;
+    p.B = batch; p.C = channels; p.T = frames; p.n_fft = n_fft; p.hop = hop; p.win = win;
+    p.out_len = (int)out_len;
+    p.R = R; p.seg = best_seg; p.n_warps = NW;
+    p.n_tiles_t = (int)((hops + best_seg - 1) / best_seg);
+    const long long tiles = (long long)batch * channels * p.n_tiles_t;
+    if (tiles > 0x7fffffffLL) return kb_fail(KAPRE_E_UNSUPPORTED, "too many tiles");
+    const int grid = (int)(tiles < slots ? tiles : slots);
+    {
+        char buf[160];
+        snprintf(buf, sizeof(buf), "ISTFT2 Q%d NW%d seg%d rounds%d tiles%lld grid%d smem%d bps%d", Q, NW, best_seg, best_m, tiles, grid, L2.total, bps);
+        g_launch_info = buf;
+    }
+    *grid_out = grid;
+    return 0;
+}
+
+template <bool ADJ>
+static int kb_launch_istft2_q(int Q, const KbIstftParams& p, int grid, cudaStream_t st) {
+    const int smem = kb_istft2_smem_layout(Q, p.n_fft, p.hop, p.win, p.n_warps).total;
+    switch (Q) {
+        case 4: return kb_launch_istft2<4, ADJ>(p, grid, smem, st);
+        case 8: return kb_launch_istft2<8, ADJ>(p, grid, smem, st);
+        case 16: return kb_launch_istft2<16, ADJ>(p, grid, smem, st);
+        case 32: return kb_launch_istft2<32, ADJ>(p, grid, smem, st);
+        default: return kb_fail(KAPRE_E_UNSUPPORTED, "bad Q");
+    }
 }
 
 
@@ -896,12 +1000,31 @@ int kapre_stft_plan_create(int n_fft, int win_length, int hop_length, const floa
         }
         if ((rc = kb_upload(w, &p->w)) || (rc = kb_upload(tw, &p->tw))) { kapre_stft_plan_destroy(p); return rc; }
     }
+    {   // adjoint tables
+        std::vector<float> wa(p->win_eff), dn(p->win_eff);
+        for (int m = 0; m < p->win_eff; ++m) {
+            wa[m] = (float)(0.5 * (double)n_fft * (double)window_host[m]);
+            dn[m] = (float)(0.5 * (double)window_host[m]);
+        }
+        std::vector<float2> tw(n_fft);
+        for (int r = 0; r < n_fft; ++r) {
+            const double a = 2.0 * M_PI * (double)r / (double)n_fft;
+            tw[r] = make_float2((float)cos(a), (float)sin(a));
+        }
+        if ((rc = kb_upload(dn, &p->adj_dn)) || (rc = kb_upload(tw, &p->adj_tw))) { kapre_stft_plan_destroy(p); return rc; }
+        if (p->Q) {
+            std::vector<float> adj;
+            kb_make_dual(wa.data(), p->win_eff, n_fft, adj);
+            if ((rc = kb_upload(adj, &p->adj))) { kapre_stft_plan_destroy(p); return rc; }
+        }
+    }
     *out = p;
     return 0;
 }
 
 void kapre_stft_plan_destroy(kapre_stft_plan* p) {
     if (!p) return;
+    cudaFree(p->adj); cudaFree(p->adj_dn); cudaFree(p->adj_tw);
     cudaFree(p->wh); cudaFree(p->cwq); cudaFree(p->twp); cudaFree(p->twn); cudaFree(p->twn2); cudaFree(p->w); cudaFree(p->tw);
     cudaFree(p->tc_f1); cudaFree(p->tc_cs); cudaFree(p->tc_csb); cudaFree(p->tc_tw); cudaFree(p->tc_w32);
     delete p;
@@ -1250,6 +1373,11 @@ int kapre_istft_plan_create(int n_fft, int win_length, int hop_length, const flo
         }
         if ((rc = kb_upload(dn, &p->dualn)) || (rc = kb_upload(tw, &p->tw))) { kapre_istft_plan_destroy(p); return rc; }
     }
+    {   // VJP: the forward STFT of the upstream gradient with the window 2/n_fft * dual (kapre_istft_backward)
+        std::vector<float> w2(win_length);
+        for (int m = 0; m < win_length; ++m) w2[m] = (float)(2.0 * (double)dual_window_host[m] / (double)n_fft);
+        if ((rc = kapre_stft_plan_create(n_fft, win_length, hop_length, w2.data(), &p->grad))) { kapre_istft_plan_destroy(p); return rc; }
+    }
     *out = p;
     return 0;
 }
@@ -1257,6 +1385,7 @@ int kapre_istft_plan_create(int n_fft, int win_length, int hop_length, const flo
 void kapre_istft_plan_destroy(kapre_istft_plan* p) {
     if (!p) return;
     cudaFree(p->dual); cudaFree(p->twp); cudaFree(p->twn); cudaFree(p->dualn); cudaFree(p->tw);
+    kapre_stft_plan_destroy(p->grad);
     delete p;
 }
 
@@ -1295,55 +1424,15 @@ int kapre_istft_inverse(const kapre_istft_plan* plan, const void* stft_dev, int 
     const int Q = plan->Q, FPW = 32 / Q;
     const int R = (plan->win + plan->hop - 1) / plan->hop;
     if (kb_env_int("KAPRE_B200_ISTFT2", 1)) {
-        // streaming kernel: tiles of seg = m * FR - (R - 1) output hops, m rounds of FR = NW * FPW frames each.  m is the
-        // round count that minimises (waves of tiles over the resident CTAs) x (rounds per tile).
-        const int NW = KB_ISTFT_MAX_WARPS, FR = NW * FPW;
-        const KbIstft2Smem L2 = kb_istft2_smem_layout(Q, plan->n_fft, plan->hop, plan->win, NW);
-        if (L2.total <= plan->dev.smem_optin) {
-            int bps = (228 * 1024) / (L2.total + 1024);
-            if (bps > 4) bps = 4;              // __launch_bounds__(128, 4)
-            if (bps < 1) bps = 1;
-            const long long slots = (long long)plan->dev.sm_count * bps;
-            const long long hops = (out_len + plan->hop - 1) / plan->hop;
-            // rounds per tile: the most (<= 6: R - 1 halo frames per tile cost <= 6 %) that still leave about one tile per
-            // resident CTA.  Measured (profiles/r2_istft_streaming.md): at B256 x 5 s tiles of 6 rounds beat one wave of 28-round
-            // tiles by 6 % (the static tile walk balances per SM, not per CTA); at B128 x 1 s tiles of 3 rounds (512 tiles on
-            // 592 slots) beat 2 and 4.
-            // Floor: tiles long enough that the halo stays under ~20 % of the frames (hop << win: R is large).
-            int m_lo = (5 * (R - 1) + FR - 1) / FR;
-            if (m_lo < 1) m_lo = 1;
-            const int m_hi = m_lo > 6 ? m_lo : 6;
-            int best_m = m_lo, best_seg = m_lo * FR - (R - 1);
-            for (int m = m_hi; m >= m_lo; --m) {
-                const int seg = m * FR - (R - 1);
-                const long long nt = (long long)batch * channels * ((hops + seg - 1) / seg);
-                best_m = m; best_seg = seg;
-                if (nt * 100 >= slots * 85) break;
-            }
-            const int m_env = kb_env_int("KAPRE_B200_ISTFT2_M", 0);
-            if (m_env > 0 && m_env * FR - (R - 1) >= 1) { best_m = m_env; best_seg = m_env * FR - (R - 1); }
-            KbIstftParams p{};
+        KbIstftParams p{};
+        int grid = 0;
+        if ((rc = kb_istft2_cfg(plan->dev, Q, plan->n_fft, plan->hop, plan->win, batch, channels, frames, out_len, &p, &grid)) < 0)
+            return rc;
+        if (rc == 0) {
             p.X = (const float2*)stft_dev; p.x_sb = sd->stride_b; p.x_sc = sd->stride_c; p.x_st = sd->stride_t; p.x_sk = sd->stride_f;
-            p.B = batch; p.C = channels; p.T = frames; p.n_fft = plan->n_fft; p.hop = plan->hop; p.win = plan->win;
-            p.out_len = (int)out_len; p.dual = plan->dual; p.twp = plan->twp; p.twn = plan->twn;
+            p.dual = plan->dual; p.twp = plan->twp; p.twn = plan->twn;
             p.y = y_dev; p.y_sb = yd->stride_b; p.y_sc = yd->stride_c; p.y_sl = yd->stride_l;
-            p.R = R; p.seg = best_seg; p.n_warps = NW;
-            p.n_tiles_t = kb_istft2_tiles(frames, plan->hop, plan->win_length, best_seg);
-            const long long tiles = (long long)batch * channels * p.n_tiles_t;
-            if (tiles > 0x7fffffffLL) return kb_fail(KAPRE_E_UNSUPPORTED, "too many tiles");
-            const int grid = (int)(tiles < slots ? tiles : slots);
-            {
-                char buf[160];
-                snprintf(buf, sizeof(buf), "ISTFT2 Q%d NW%d seg%d rounds%d tiles%lld grid%d smem%d bps%d", Q, NW, best_seg, best_m, tiles, grid, L2.total, bps);
-                g_launch_info = buf;
-            }
-            switch (Q) {
-                case 4: return kb_launch_istft2<4>(p, grid, L2.total, st);
-                case 8: return kb_launch_istft2<8>(p, grid, L2.total, st);
-                case 16: return kb_launch_istft2<16>(p, grid, L2.total, st);
-                case 32: return kb_launch_istft2<32>(p, grid, L2.total, st);
-                default: return kb_fail(KAPRE_E_UNSUPPORTED, "bad Q");
-            }
+            return kb_launch_istft2_q<false>(Q, p, grid, st);
         }
     }
     // one FFT round per overlap class: TFc = R * NW * FPW frames per tile
@@ -1393,6 +1482,14 @@ int kapre_filterbank_create(const float* fb_host, int n_freq, int n_bands, kapre
     kb_make_bands(fb_host, n_freq, n_bands, bands, w);
     f->n_w = (int)w.size();
     if ((rc = kb_upload(bands, &f->bands)) || (rc = kb_upload(w, &f->w))) { kapre_filterbank_destroy(f); return rc; }
+    {   // transposed form for the spectral VJP (g_mag = g_fb fb^T)
+        std::vector<float> fbT((size_t)n_freq * n_bands);
+        for (int k = 0; k < n_freq; ++k)
+            for (int m = 0; m < n_bands; ++m) fbT[(size_t)m * n_freq + k] = fb_host[(size_t)k * n_bands + m];
+        std::vector<KbBand> bT; std::vector<float> wT;
+        kb_make_bands(fbT.data(), n_bands, n_freq, bT, wT);
+        if ((rc = kb_upload(bT, &f->bandsT)) || (rc = kb_upload(wT, &f->wT))) { kapre_filterbank_destroy(f); return rc; }
+    }
     f->Q = kb_q_for_nfft((n_freq - 1) * 2);
     if (f->Q) {
         std::vector<kb_f4> cw; std::vector<kb_i2> cm; std::vector<int> cg;
@@ -1418,7 +1515,7 @@ int kapre_filterbank_create(const float* fb_host, int n_freq, int n_bands, kapre
 
 void kapre_filterbank_destroy(kapre_filterbank* f) {
     if (!f) return;
-    cudaFree(f->bands); cudaFree(f->w); cudaFree(f->cw); cudaFree(f->cm); cudaFree(f->cg);
+    cudaFree(f->bands); cudaFree(f->w); cudaFree(f->bandsT); cudaFree(f->wT); cudaFree(f->cw); cudaFree(f->cm); cudaFree(f->cg);
     cudaFree(f->mw); cudaFree(f->ms); cudaFree(f->mg); cudaFree(f->bd); cudaFree(f->bg);
     delete f;
 }
@@ -1659,4 +1756,204 @@ int kapre_tc_dft_stage1(const float* x_dev, int n_items, long long item_stride, 
     return 0;
 }
 
+// ---- backward (vector-Jacobian products), grad_core.cuh -----------------------------------------------------------
+// Workspace of the decibel statistics: [arrival counters, n_items words | pad to 16 B][stats, 16 B per item]
+// [partials, KB_DBS_MAX_CHUNKS * 16 B per item]
+static void kb_dbs_ws(void* ws, long long n_items, unsigned int** arrive, KbDbStats** stats, KbDbStats** part) {
+    char* base = (char*)ws;
+    const long long a = (n_items * 4 + 15) & ~15LL;
+    *arrive = (unsigned int*)base;
+    *stats = (KbDbStats*)(base + a);
+    *part = (KbDbStats*)(base + a + n_items * (long long)sizeof(KbDbStats));
+}
+
+// Statistics pass over a (n_items, d1, d2, d3) view of y and g; leaves the combined KbDbStats per item in the workspace.
+static int kb_launch_dbstat(KbDbStatParams& q, void* ws, float dyn_range, cudaStream_t st, KbDbStats** stats_out) {
+    const long long item = (long long)q.d1 * q.d2 * q.d3;
+    long long chunks = (item + 32767) / 32768;
+    if (chunks > KB_DBS_MAX_CHUNKS) chunks = KB_DBS_MAX_CHUNKS;
+    if (chunks < 1) chunks = 1;
+    if ((long long)q.n_items * chunks > 0x7fffffffLL) return kb_fail(KAPRE_E_UNSUPPORTED, "too many items");
+    q.chunks = (int)chunks;
+    q.dyn_range = dyn_range;
+    KbDbStats* part;
+    kb_dbs_ws(ws, q.n_items, &q.arrive, &q.stats, &part);
+    q.part = part;
+    kb_dbstat_kernel<<<(unsigned)(q.n_items * chunks), KB_DBS_THREADS, 0, st>>>(q);
+    KB_CUDA(cudaGetLastError());
+    g_launches++;
+    *stats_out = q.stats;
+    return 0;
+}
+
+int kapre_stft_backward(const kapre_stft_plan* plan, const void* grad_spec_dev, int batch, int channels, int frames,
+                        const kapre_spec_desc* gsd, int pad_begin, int pad_end, float* grad_x_dev,
+                        const kapre_wave_desc* gxd, void* stream) {
+    if (!plan || !gsd || !gxd) return kb_fail(KAPRE_E_INVALID, "null argument");
+    int rc = kb_check_device(plan->dev);
+    if (rc) return rc;
+    if (batch < 0 || channels < 0 || frames < 0 || gxd->length < 0) return kb_fail(KAPRE_E_INVALID, "negative size");
+    if (gxd->batch != batch || gxd->channels != channels)
+        return kb_fail(KAPRE_E_INVALID, "gradient is (%d, %d) signals, the spectrum (%d, %d)", gxd->batch, gxd->channels, batch, channels);
+    if (pad_begin && plan->hop > plan->n_fft)
+        return kb_fail(KAPRE_E_INVALID, "pad_begin needs hop_length <= n_fft (the padding is n_fft - hop_length = %d)",
+                       plan->n_fft - plan->hop);
+    const int L = gxd->length;
+    const int T = kapre_stft_num_frames(plan, L, pad_begin, pad_end);
+    if (T != frames) return kb_fail(KAPRE_E_INVALID, "%d samples give %d frames, the spectrum has %d", L, T, frames);
+    if (batch == 0 || channels == 0 || L == 0) return 0;
+    if (!grad_x_dev || (frames > 0 && !grad_spec_dev)) return kb_fail(KAPRE_E_INVALID, "null data pointer");
+    const int pad_left = pad_begin ? (plan->n_fft - plan->hop) : 0;
+    const long long out_len = (long long)pad_left + L;      // padded coordinates; [0, pad_left) is dropped
+    if (out_len + plan->n_fft > 0x7fffffffLL) return kb_fail(KAPRE_E_UNSUPPORTED, "signal too long");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (plan->Q && frames > 0 && kb_env_int("KAPRE_B200_ISTFT2", 1)) {
+        KbIstftParams p{};
+        int grid = 0;
+        if ((rc = kb_istft2_cfg(plan->dev, plan->Q, plan->n_fft, plan->hop, plan->win_eff, batch, channels, frames, out_len,
+                                &p, &grid)) < 0)
+            return rc;
+        if (rc == 0) {
+            p.X = (const float2*)grad_spec_dev; p.x_sb = gsd->stride_b; p.x_sc = gsd->stride_c; p.x_st = gsd->stride_t;
+            p.x_sk = gsd->stride_f;
+            p.dual = plan->adj; p.twp = plan->twp; p.twn = plan->twn;
+            p.y = grad_x_dev; p.y_sb = gxd->stride_b; p.y_sc = gxd->stride_c; p.y_sl = gxd->stride_l;
+            p.y_off = pad_left; p.edge2 = 1;
+            return kb_launch_istft2_q<true>(plan->Q, p, grid, st);
+        }
+    }
+    // direct body: every n_fft, O(n_fft) work per output sample and frame (also zero-fills when there are no frames)
+    KbIdftParams p{};
+    p.X = (const float2*)grad_spec_dev; p.x_sb = gsd->stride_b; p.x_sc = gsd->stride_c; p.x_st = gsd->stride_t; p.x_sk = gsd->stride_f;
+    p.B = batch; p.C = channels; p.T = frames; p.n_fft = plan->n_fft; p.hop = plan->hop; p.win = plan->win_eff;
+    p.out_len = (int)out_len; p.dualn = plan->adj_dn; p.tw = plan->adj_tw;
+    p.y = grad_x_dev; p.y_sb = gxd->stride_b; p.y_sc = gxd->stride_c; p.y_sl = gxd->stride_l;
+    p.y_off = pad_left; p.edge2 = 1;
+    p.n_warps = 8; p.n_tiles_s = (int)((out_len + 255) / 256);
+    const int smem = plan->n_fft * 8;
+    if (smem > plan->dev.smem_optin) return kb_fail(KAPRE_E_UNSUPPORTED, "n_fft too large");
+    if ((rc = kb_set_smem(kb_idft_kernel, smem))) return rc;
+    const long long tiles = (long long)batch * channels * p.n_tiles_s;
+    if (tiles > 0x7fffffffLL) return kb_fail(KAPRE_E_UNSUPPORTED, "too many tiles");
+    const int grid = (int)(tiles < plan->dev.sm_count * 8LL ? tiles : plan->dev.sm_count * 8LL);
+    kb_idft_kernel<<<grid, 256, smem, st>>>(p);
+    KB_CUDA(cudaGetLastError());
+    g_launches++;
+    return 0;
+}
+
+int kapre_istft_backward(const kapre_istft_plan* plan, const float* grad_y_dev, const kapre_wave_desc* gyd,
+                         void* grad_spec_dev, int frames, const kapre_spec_desc* gsd, void* stream) {
+    if (!plan || !gyd || !gsd) return kb_fail(KAPRE_E_INVALID, "null argument");
+    int rc = kb_check_device(plan->dev);
+    if (rc) return rc;
+    if (gyd->batch < 0 || gyd->channels < 0 || frames < 0) return kb_fail(KAPRE_E_INVALID, "negative size");
+    if (gyd->batch == 0 || gyd->channels == 0 || frames == 0) return 0;
+    const long long out_len = (long long)(frames - 1) * plan->hop + plan->win_length;
+    if (gyd->length != out_len)
+        return kb_fail(KAPRE_E_INVALID, "gradient length must be (frames-1)*hop+win_length = %lld, got %d", out_len, gyd->length);
+    if (!grad_y_dev || !grad_spec_dev) return kb_fail(KAPRE_E_INVALID, "null data pointer");
+    if ((rc = kapre_stft_forward(plan->grad, grad_y_dev, gyd, 0, 0, KAPRE_OUT_COMPLEX, grad_spec_dev, gsd, nullptr, nullptr,
+                                 nullptr, stream)))
+        return rc;
+    const long long n_frames = (long long)gyd->batch * gyd->channels * frames;
+    int grid = 0;
+    if ((rc = kb_ew_grid(n_frames, &grid))) return rc;
+    kb_istft_grad_edges_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((float2*)grad_spec_dev, gsd->stride_b, gsd->stride_c,
+                                                                       gsd->stride_t, gsd->stride_f, gyd->channels, frames,
+                                                                       n_frames, plan->n_fft / 2, (plan->n_fft & 1) == 0);
+    KB_CUDA(cudaGetLastError());
+    g_launches++;
+    return 0;
+}
+
+int kapre_spectral_backward(const kapre_filterbank* fb, int mode, const void* x_dev, int batch, int channels, int frames,
+                            int n_freq, const kapre_spec_desc* xd, const float* grad_dev, const kapre_spec_desc* gd,
+                            const float* y_dev, const kapre_spec_desc* yd, const kapre_db_cfg* db, void* workspace_dev,
+                            void* grad_x_dev, const kapre_spec_desc* gxd, void* stream) {
+    if (!xd || !gd || !gxd) return kb_fail(KAPRE_E_INVALID, "null argument");
+    if (mode != KAPRE_OUT_MAG && mode != KAPRE_OUT_MAG_DB && mode != KAPRE_OUT_FB && mode != KAPRE_OUT_FB_DB)
+        return kb_fail(KAPRE_E_INVALID, "bad mode %d for the spectral VJP", mode);
+    if (batch < 0 || channels < 0 || frames < 0 || n_freq < 1) return kb_fail(KAPRE_E_INVALID, "bad size");
+    const bool fbm = mode == KAPRE_OUT_FB || mode == KAPRE_OUT_FB_DB;
+    const bool dbm = mode == KAPRE_OUT_MAG_DB || mode == KAPRE_OUT_FB_DB;
+    int rc = 0;
+    if (fbm) {
+        if (!fb) return kb_fail(KAPRE_E_INVALID, "filterbank required for mode %d", mode);
+        if (fb->n_freq != n_freq) return kb_fail(KAPRE_E_INVALID, "filterbank has %d rows, the spectrum %d bins", fb->n_freq, n_freq);
+        if ((rc = kb_check_device(fb->dev))) return rc;
+    }
+    if (dbm) {
+        if ((rc = kb_check_db(db))) return rc;
+        if (!yd) return kb_fail(KAPRE_E_INVALID, "forward output required for decibel modes");
+        if (!workspace_dev) return kb_fail(KAPRE_E_INVALID, "workspace required for decibel modes");
+    }
+    if (batch == 0 || channels == 0 || frames == 0) return 0;
+    if (!x_dev || !grad_dev || !grad_x_dev || (dbm && !y_dev)) return kb_fail(KAPRE_E_INVALID, "null data pointer");
+    const int K = fbm ? fb->n_bands : n_freq;
+    cudaStream_t st = (cudaStream_t)stream;
+    DevInfo dev;
+    if ((rc = kb_dev_info(&dev))) return rc;
+    KbSpecVjpParams p{};
+    if (dbm) {
+        KbDbStatParams q{};
+        q.y = y_dev; q.y_s0 = yd->stride_b; q.y_s1 = yd->stride_c; q.y_s2 = yd->stride_t; q.y_s3 = yd->stride_f;
+        q.g = grad_dev; q.g_s0 = gd->stride_b; q.g_s1 = gd->stride_c; q.g_s2 = gd->stride_t; q.g_s3 = gd->stride_f;
+        q.n_items = batch; q.d1 = channels; q.d2 = frames; q.d3 = K;
+        KbDbStats* stats = nullptr;
+        if ((rc = kb_launch_dbstat(q, workspace_dev, db->dynamic_range, st, &stats))) return rc;
+        p.stats = stats;
+        p.amin = db->amin;
+        p.y = y_dev; p.y_sb = yd->stride_b; p.y_sc = yd->stride_c; p.y_st = yd->stride_t; p.y_sk = yd->stride_f;
+    }
+    p.X = (const float2*)x_dev; p.x_sb = xd->stride_b; p.x_sc = xd->stride_c; p.x_st = xd->stride_t; p.x_sk = xd->stride_f;
+    p.G = (float2*)grad_x_dev; p.G_sb = gxd->stride_b; p.G_sc = gxd->stride_c; p.G_st = gxd->stride_t; p.G_sk = gxd->stride_f;
+    p.g = grad_dev; p.g_sb = gd->stride_b; p.g_sc = gd->stride_c; p.g_st = gd->stride_t; p.g_sk = gd->stride_f;
+    p.B = batch; p.C = channels; p.T = frames; p.F = n_freq; p.K = K;
+    p.fb = fbm; p.db = dbm;
+    if (fbm) { p.bands = fb->bands; p.fbw = fb->w; p.bandsT = fb->bandsT; p.fbwT = fb->wT; }
+    p.n_warps = 4;
+    const int smem = kb_specvjp_smem_layout(n_freq, K).total;
+    if (smem > dev.smem_optin) return kb_fail(KAPRE_E_UNSUPPORTED, "spectrum of %d bins does not fit shared memory", n_freq);
+    if ((rc = kb_set_smem(kb_specvjp_kernel, smem))) return rc;
+    int bps = (228 * 1024) / (smem + 1024);
+    if (bps > 16) bps = 16;
+    if (bps < 1) bps = 1;
+    const long long n_frames = (long long)batch * channels * frames;
+    const long long gmax = (long long)dev.sm_count * bps;
+    const int grid = (int)(n_frames < gmax ? n_frames : gmax);
+    kb_specvjp_kernel<<<grid, p.n_warps * 32, smem, st>>>(p);
+    KB_CUDA(cudaGetLastError());
+    g_launches++;
+    return 0;
+}
+
+int kapre_magnitude_to_decibel_backward(const float* x_dev, const float* y_dev, const float* grad_dev,
+                                        int64_t grad_item_stride, int64_t grad_elem_stride, float* grad_x_dev,
+                                        int64_t n_items, int64_t item_size, const kapre_db_cfg* db, void* workspace_dev,
+                                        void* stream) {
+    int rc = kb_check_db(db);
+    if (rc) return rc;
+    if (n_items < 0 || item_size < 0) return kb_fail(KAPRE_E_INVALID, "negative size");
+    if (n_items == 0 || item_size == 0) return 0;
+    if (!x_dev || !y_dev || !grad_dev || !grad_x_dev || !workspace_dev) return kb_fail(KAPRE_E_INVALID, "null pointer");
+    if (n_items > 0x7fffffffLL || item_size > 0x7fffffffLL) return kb_fail(KAPRE_E_UNSUPPORTED, "tensor too large");
+    cudaStream_t st = (cudaStream_t)stream;
+    KbDbStatParams q{};
+    q.y = y_dev; q.y_s0 = item_size; q.y_s1 = 0; q.y_s2 = 0; q.y_s3 = 1;
+    q.g = grad_dev; q.g_s0 = grad_item_stride; q.g_s1 = 0; q.g_s2 = 0; q.g_s3 = grad_elem_stride;
+    q.n_items = (int)n_items; q.d1 = 1; q.d2 = 1; q.d3 = (int)item_size;
+    KbDbStats* stats = nullptr;
+    if ((rc = kb_launch_dbstat(q, workspace_dev, db->dynamic_range, st, &stats))) return rc;
+    const long long n = n_items * item_size;
+    int grid = 0;
+    if ((rc = kb_ew_grid(n, &grid))) return rc;
+    kb_db_backward_kernel<<<grid, 256, 0, st>>>(x_dev, y_dev, grad_dev, grad_item_stride, grad_elem_stride, grad_x_dev,
+                                                item_size, n, stats, db->amin);
+    KB_CUDA(cudaGetLastError());
+    g_launches++;
+    return 0;
+}
+
 }  // extern "C"
+

@@ -130,6 +130,10 @@ struct KbIstftParams {
     int n_tiles_t;
     int n_warps;
     int seg;                             // streaming kernel (kb_istft2_cta): output hops per tile
+    // STFT adjoint (kapre_stft_backward) only; zero for the inverse STFT.  y_off: output sample s goes to y[s - y_off]
+    // and samples below y_off are dropped (the pad_begin prefix); edge2: Re X[0] and Re X[N/2] are doubled at load.
+    int y_off;
+    int edge2;
 };
 
 // Complex number = one aligned register pair.  On sm_100a the arithmetic below compiles to the

@@ -466,3 +466,130 @@ def energy(x: torch.Tensor, frame_length, hop_length, pad_end, pad_value, scale,
                                      ctypes.c_float(pad_value), ctypes.c_float(scale), _ptr(out), ctypes.byref(od),
                                      _stream_ptr()))
     return out
+
+
+# ------------------------------------------------------------------------------- backward (VJPs)
+def grad_workspace(n_items: int, device) -> torch.Tensor:
+    """Zeroed scratch of the decibel VJP statistics (C ABI: >= 1056 * n_items + 16 bytes, zero on entry, left zero)."""
+    n = max(int(n_items), 1)
+    return torch.zeros(((n * 4 + 15) // 16 * 16 + 1040 * n) // 4, dtype=torch.int32, device=device)
+
+
+def _resolved(t: torch.Tensor) -> torch.Tensor:
+    """Materialise torch's lazy conjugate / negative views (their bits are not what the strides describe)."""
+    return t.resolve_conj().resolve_neg() if t.is_complex() else t.resolve_neg()
+
+
+def transposed(fb: Filterbank) -> Filterbank:
+    """The (n_bands, n_freq) transpose of a filterbank: ApplyFilterbank's VJP is ApplyFilterbank with it."""
+    t = getattr(fb, '_transposed', None)
+    if t is None:
+        t = fb._transposed = Filterbank(fb.matrix.T)
+    return t
+
+
+@_device_of_first_arg
+def stft_backward(G: torch.Tensor, plan: StftPlan, spec_format, wave_format, pad_begin, pad_end, length):
+    """VJP of the STFT: complex gradient of the spectrum (layout ``spec_format``) -> float32 gradient of the waveform
+    (layout ``wave_format``, ``length`` samples).  One launch of the windowed overlap-add of inverse real FFTs."""
+    if not G.is_cuda:
+        raise N.KapreNativeError('stft_backward needs a CUDA tensor')
+    G = _resolved(G.to(torch.complex64))
+    sd, (B, C, T, F) = _spec_desc(G, spec_format)
+    L = int(length)
+    if F != plan.n_fft // 2 + 1:
+        raise ValueError('expected %d frequency bins for n_fft=%d, got %d' % (plan.n_fft // 2 + 1, plan.n_fft, F))
+    if wave_format == _CH_LAST_STR:
+        gx = torch.empty((B, L, C), dtype=torch.float32, device=G.device)
+        sb, sl, sc = gx.stride()
+    else:
+        gx = torch.empty((B, C, L), dtype=torch.float32, device=G.device)
+        sb, sc, sl = gx.stride()
+    if gx.numel():
+        xd = N.WaveDesc(B, C, L, sb, sc, sl)
+        N.check(N.lib().kapre_stft_backward(plan.handle(), _ptr(G), B, C, T, ctypes.byref(sd), int(bool(pad_begin)),
+                                            int(bool(pad_end)), _ptr(gx), ctypes.byref(xd), _stream_ptr()))
+    return gx
+
+
+@_device_of_first_arg
+def istft_backward(gy: torch.Tensor, plan: IstftPlan, spec_format, wave_format, frames):
+    """VJP of the inverse STFT: float gradient of the waveform -> complex64 gradient of the ``frames``-frame spectrum."""
+    if not gy.is_cuda:
+        raise N.KapreNativeError('istft_backward needs a CUDA tensor')
+    gy = _resolved(gy.to(torch.float32))
+    yd, (B, C, L) = _wave_desc(gy, wave_format)
+    G, gd = _spec_alloc(B, C, int(frames), plan.n_fft // 2 + 1, spec_format, torch.complex64, gy.device)
+    if G.numel():
+        N.check(N.lib().kapre_istft_backward(plan.handle(), _ptr(gy), ctypes.byref(yd), _ptr(G), int(frames),
+                                             ctypes.byref(gd), _stream_ptr()))
+    return G
+
+
+@_device_of_first_arg
+def spectral_backward(X: torch.Tensor, g: torch.Tensor, y, mode, fb: Filterbank, db, data_format, out=None):
+    """VJP of |.| [-> filterbank] [-> dB] at the complex STFT ``X`` (4-D, ``data_format``): upstream gradient ``g`` and,
+    for the decibel modes, forward output ``y`` (both (B, C, T, K) in ``data_format``) -> complex gradient of ``X``.
+    ``out`` may be ``X`` itself (in place)."""
+    if not X.is_cuda:
+        raise N.KapreNativeError('spectral_backward needs a CUDA tensor')
+    if X.dtype != torch.complex64:
+        raise ValueError('spectral_backward needs a complex64 spectrum')
+    xd, (B, C, T, F) = _spec_desc(X, data_format)
+    g = _resolved(g.to(torch.float32))
+    gd, _ = _spec_desc(g, data_format)
+    fbmode = mode in (N.OUT_FB, N.OUT_FB_DB)
+    dbmode = mode in (N.OUT_MAG_DB, N.OUT_FB_DB)
+    if out is None:
+        out, od = _spec_alloc(B, C, T, F, data_format, torch.complex64, X.device)
+    else:
+        od, _ = _spec_desc(out, data_format)
+    yd, dbc, ws = None, None, None
+    if dbmode:
+        yd, _ = _spec_desc(y, data_format)
+        dbc = N.DbCfg(float(db[0]), float(db[1]), float(db[2]))
+        ws = grad_workspace(B, X.device)
+    if out.numel():
+        N.check(N.lib().kapre_spectral_backward(
+            fb.handle() if fbmode else None, int(mode), _ptr(X), B, C, T, F, ctypes.byref(xd), _ptr(g), ctypes.byref(gd),
+            _ptr(y) if dbmode else None, ctypes.byref(yd) if dbmode else None, ctypes.byref(dbc) if dbmode else None,
+            _ptr(ws) if dbmode else None, _ptr(out), ctypes.byref(od), _stream_ptr()))
+    return out
+
+
+def _items(t: torch.Tensor):
+    """(n_items, item_size) of the decibel layer: per batch item, or one item for a 1-D tensor (kapre/backend.py:178-179)."""
+    if t.dim() > 1:
+        return t.shape[0], t.numel() // t.shape[0]
+    return 1, t.numel()
+
+
+@_device_of_first_arg
+def magnitude_to_decibel_backward(x: torch.Tensor, y: torch.Tensor, g: torch.Tensor, ref_value, amin, dynamic_range):
+    """VJP of MagnitudeToDecibel: contiguous float32 input ``x`` and output ``y`` of the forward, upstream gradient ``g``
+    (any strides) -> float32 gradient of ``x``."""
+    if not x.is_cuda:
+        raise N.KapreNativeError('magnitude_to_decibel_backward needs a CUDA tensor')
+    gx = torch.empty_like(x)
+    if x.numel() == 0:
+        return gx
+    n_items, item = _items(x)
+    g2 = _resolved(g.to(torch.float32)).reshape(n_items, item)
+    ws = grad_workspace(n_items, x.device)
+    dbc = N.DbCfg(float(ref_value), float(amin), float(dynamic_range))
+    N.check(N.lib().kapre_magnitude_to_decibel_backward(_ptr(x), _ptr(y), _ptr(g2), g2.stride(0), g2.stride(1), _ptr(gx),
+                                                        n_items, item, ctypes.byref(dbc), _ptr(ws), _stream_ptr()))
+    return gx
+
+
+@_device_of_first_arg
+def magnitude_backward(X: torch.Tensor, g: torch.Tensor):
+    """VJP of Magnitude (tf.abs of a complex tensor): G = g X / |X|, 0 where |X| = 0."""
+    if not X.is_cuda:
+        raise N.KapreNativeError('magnitude_backward needs a CUDA tensor')
+    Xc = X.to(torch.complex64).contiguous()
+    F = Xc.shape[-1] if Xc.dim() else 1
+    X2 = Xc.reshape(1, 1, -1, F)
+    g2 = _resolved(g.to(torch.float32)).reshape(1, 1, -1, F)
+    # a (rows, F) tensor is a (1, 1, rows, F) channels_first spectrogram
+    return spectral_backward(X2, g2, None, N.OUT_MAG, None, None, _CH_FIRST_STR).reshape(Xc.shape)

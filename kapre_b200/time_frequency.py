@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from . import backend, ops
+from . import autograd, backend, ops
 from .backend import _CH_DEFAULT_STR, _CH_FIRST_STR, _CH_LAST_STR
 
 __all__ = ['Layer', 'STFT', 'InverseSTFT', 'Magnitude', 'Phase', 'MagnitudeToDecibel', 'ApplyFilterbank', 'Delta']
@@ -152,6 +152,8 @@ class STFT(Layer):
         return self._plan
 
     def call(self, x):
+        if autograd.wants_grad(x):
+            return autograd.StftFn.apply(x, self)
         return ops.stft_forward(x, self.plan, self.input_data_format, self.output_data_format,
                                 self.pad_begin, self.pad_end, N.OUT_COMPLEX)
 
@@ -208,6 +210,8 @@ class InverseSTFT(Layer):
         return self._plan
 
     def call(self, x):
+        if autograd.wants_grad(x):
+            return autograd.IstftFn.apply(x, self)
         return ops.istft(x, self.plan, self.input_data_format, self.output_data_format)
 
     _config_fields = (
@@ -225,6 +229,8 @@ class Magnitude(Layer):
     """``tf.abs`` of the complex input (reference: kapre/time_frequency.py:337-359)."""
 
     def call(self, x):
+        if autograd.wants_grad(x) and x.is_complex():
+            return autograd.MagnitudeFn.apply(x)
         return ops.magnitude(x)
 
 
@@ -256,6 +262,8 @@ class MagnitudeToDecibel(Layer):
         self.dynamic_range = dynamic_range
 
     def call(self, x):
+        if autograd.wants_grad(x):
+            return autograd.MagnitudeToDecibelFn.apply(x, self.ref_value, self.amin, self.dynamic_range)
         return backend.magnitude_to_decibel(x, ref_value=self.ref_value, amin=self.amin,
                                             dynamic_range=self.dynamic_range)
 
@@ -290,6 +298,8 @@ class ApplyFilterbank(Layer):
         return self._fb
 
     def call(self, x):
+        if autograd.wants_grad(x):
+            return autograd.ApplyFilterbankFn.apply(x, self)
         return ops.apply_filterbank(x, self.fb, self.data_format)
 
     _config_fields = (
